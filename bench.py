@@ -23,6 +23,9 @@ A "step" = one pass of solve() over this rank's batch.
   latency : one problem through tzr_solve (the drop-in solve() shape), p50 over >= 20 calls.
 Inputs per step are larger than L2 for the batch configs; for the small ones an L2 flush (256 MB write) runs
 between steps and is excluded from the per-stage kernel times but not from ms_per_step — see config.l2.
+
+--dump-outputs DIR writes what the last timed step returned as DIR/<name>.npy (see dump_outputs), so that two builds
+run with the same arguments, and therefore on the same seeded inputs, can be compared output for output.
 """
 import argparse
 import importlib
@@ -138,6 +141,35 @@ def solver_params(mod, cfg, nb, estimate_scaling):
                               inlier_selection_mode=0)
 
 
+DUMP_BUDGET_BYTES = 63_000_000  # array data; leaves room for the .npy headers under 64 MB in all
+# every solution field except stage_ms, which holds timings rather than results
+DUMP_FIELDS = ("valid", "clique_size", "scale", "translation", "rotation", "clique_proven_optimal", "gnc_iterations",
+               "gnc_cost", "n_rotation_inliers", "n_translation_inliers", "n_edges")
+
+
+def dump_outputs(out_dir, sols, clq, problems):
+    """Writes one step's results of tzr_solve_batch_dev as out_dir/<name>.npy: each field of DUMP_FIELDS in float64
+    (rotation as (B, 3, 3) matrices, gnc_cost -1 where the record holds +inf), clique (B, N) float32 with the clique's
+    indices and -1 past clique_size, and problem, the synth problem number of each row.  Every value is finite.  A batch
+    over DUMP_BUDGET_BYTES is cut to a sample of rows drawn with a fixed seed from the batch shape alone, so that every
+    build dumps the same problems."""
+    B, n = clq.shape
+    per_problem = 4 * n + 8 * (1 + sum(int(np.prod(sols.dtype[f].shape)) for f in DUMP_FIELDS))
+    keep = DUMP_BUDGET_BYTES // per_problem
+    rows = np.arange(B) if keep >= B else np.sort(np.random.default_rng(0).choice(B, size=keep, replace=False))
+    sols, clq = sols[rows], clq[rows]
+    arrays = {f: sols[f].astype(np.float64) for f in DUMP_FIELDS}
+    arrays["rotation"] = arrays["rotation"].reshape(-1, 3, 3).transpose(0, 2, 1)  # records are column-major
+    # GNC-TLS reports +inf when it stops before its first cost evaluation (every squared residual below half the squared
+    # noise bound, registration.cc:791-792,814-825); costs are sums of squares, so -1 marks that case in a finite array
+    arrays["gnc_cost"][np.isposinf(arrays["gnc_cost"])] = -1.0
+    arrays["clique"] = np.where(np.arange(n) < sols["clique_size"][:, None], clq, -1).astype(np.float32)
+    arrays["problem"] = np.asarray(problems, dtype=np.float64)[rows]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(a))
+
+
 def workload_string(cfg, estimate_scaling, extra=""):
     sc = "unknown scale (estimate_scaling=true, the Params default)" if estimate_scaling else "fixed scale"
     return f"{CONFIGS[cfg]['desc']}, {sc}, GNC-TLS, PMC_EXACT{extra}"
@@ -228,6 +260,8 @@ def main():
     ap.add_argument("--ref-problems-per-step", type=int, default=2)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--parity-problems", type=int, default=16)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's results to DIR/<name>.npy "
+                                                          "(DIR/rank<r>/ when several ranks run)")
     args = ap.parse_args()
     if CONFIGS[args.config].get("estimate_scaling"):
         args.estimate_scaling = True
@@ -342,6 +376,9 @@ def main():
     ctx.stage_log(False)
     barrier()
     launches = ctx.kernel_launches() - l0
+    if args.dump_outputs:  # sol_d / clq_d hold the last timed step's results; nothing after this writes them
+        dump_sols = np.frombuffer(sol_d.cpu().numpy().tobytes(), dtype=capi.SOLUTION_DTYPE)
+        dump_clq = clq_d.cpu().numpy()
     t_flush = 0.0
     if flush is not None:  # the flush writes are inside ev_begin..ev_end: measure them alone and take them out
         with torch.cuda.stream(stream):
@@ -382,6 +419,9 @@ def main():
         lat.append((time.perf_counter() - t0) * 1e3)
     lat_stage = ctx.last_stage_ms()
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs if world == 1 else os.path.join(args.dump_outputs, f"rank{rank}"),
+                     dump_sols, dump_clq, idx)
 
     tt = torch.tensor([t_dev_net, t_e2e, t_pg], dtype=torch.float64, device="cuda")
     if use_dist:

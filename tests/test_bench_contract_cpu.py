@@ -46,6 +46,49 @@ def test_cuda_arm_refuses_to_run_without_a_device():
     assert not any(l.startswith("{") for l in out.stdout.splitlines())  # no number is printed
 
 
+def _fake_records(B, n, rng):
+    import numpy as np
+    capi = importlib.import_module("teaser-plusplus_b200.capi")
+    sols = np.zeros(B, dtype=capi.SOLUTION_DTYPE)
+    sols["clique_size"] = rng.integers(0, n + 1, size=B)
+    sols["rotation"] = rng.normal(size=(B, 9))
+    sols["n_edges"] = rng.integers(0, 2**40, size=B)
+    sols["gnc_cost"] = np.where(rng.random(B) < 0.5, np.inf, rng.random(B))  # +inf: GNC stopped at initialisation
+    sols["stage_ms"] = 1.0
+    return sols, rng.integers(0, n, size=(B, n)).astype(np.int32)
+
+
+def test_dump_outputs_formats_and_size_cap(tmp_path):
+    import numpy as np
+    b = _bench_module()
+    rng = np.random.default_rng(3)
+    sols, clq = _fake_records(5, 7, rng)
+    b.dump_outputs(str(tmp_path / "small"), sols, clq, np.arange(5) + 100)
+    d = {f[:-4]: np.load(tmp_path / "small" / f) for f in os.listdir(tmp_path / "small")}
+    assert set(d) == set(b.DUMP_FIELDS) | {"clique", "problem"}  # stage_ms (timings) is not a result
+    assert all(a.dtype in (np.float32, np.float64) and np.isfinite(a).all() for a in d.values())
+    assert np.array_equal(d["gnc_cost"], np.where(np.isinf(sols["gnc_cost"]), -1.0, sols["gnc_cost"]))
+    assert np.array_equal(d["problem"], np.arange(5) + 100) and np.array_equal(d["n_edges"], sols["n_edges"])
+    assert np.array_equal(d["rotation"][2], sols[2]["rotation"].reshape(3, 3).T)
+    for k in range(5):
+        m = sols[k]["clique_size"]
+        assert np.array_equal(d["clique"][k, :m], clq[k, :m]) and np.all(d["clique"][k, m:] == -1)
+
+    # a batch over the budget: a seeded sample of whole rows that depends on the batch shape only, under 64 MB on disk
+    B, n = 3000, 6000
+    big = [_fake_records(B, n, np.random.default_rng(s)) for s in (4, 5)]
+    for s, (sols, clq) in enumerate(big):
+        b.dump_outputs(str(tmp_path / f"big{s}"), sols, clq, np.arange(B))
+    p0, p1 = (np.load(tmp_path / f"big{s}" / "problem.npy") for s in (0, 1))
+    assert np.array_equal(p0, p1) and 0 < len(p0) < B and np.all(np.diff(p0) > 0)
+    assert sum(os.path.getsize(tmp_path / "big0" / f) for f in os.listdir(tmp_path / "big0")) <= 64_000_000
+    rows = p0.astype(np.int64)
+    got = np.load(tmp_path / "big0" / "clique.npy")
+    assert got.shape == (len(rows), n)
+    m = big[0][0]["clique_size"][rows[0]]
+    assert np.array_equal(got[0, :m], big[0][1][rows[0], :m])
+
+
 def test_algorithmic_bytes_model_and_config_table():
     b = _bench_module()
     # SURVEY §8d / DESIGN §3.1: 48 n (points in) + 8 n ceil(n/64) (bitset rows out) + 4 n (degrees out)
