@@ -19,6 +19,14 @@
  *   - "_dev" variants take DEVICE pointers and enqueue on the context's stream without
  *     synchronising (tzr_ctx_synchronize does); the plain variants take HOST pointers and are
  *     synchronous, host<->device copies included.
+ *   - Problem size: every entry point that takes n accepts n <= 131072 correspondences (one problem's bitset is then
+ *     2 GiB) and returns TZR_ERR_TOO_LARGE above.  For n <= 32768 the clique stage runs on the whole graph.  Above,
+ *     it first finds a greedy clique of size L on the whole graph and peels the graph to its (L-1)-core, which holds
+ *     every maximum clique; PMC_EXACT then searches that core, and TZR_ERR_TOO_LARGE is returned (tzr_last_error
+ *     names the problem and the core size) when the core has more than 32768 vertices, as on dense (~15 %) inlier
+ *     graphs, where PMC_HEU and KCORE_HEU still work.  The vertex set handed to the rotation stage (the clique or
+ *     the innermost core) must have <= 32768 vertices; estimate_scaling and inlier selection NONE need n <= 32768.
+ *     In a batch, one problem over a limit fails the whole call.
  *   - A context owns one CUDA device, one stream and a growable workspace; it is not thread-safe,
  *     distinct contexts are independent.  There is NO CPU fallback: without a usable CUDA device
  *     tzr_ctx_create fails with TZR_ERR_NO_DEVICE.
@@ -229,7 +237,9 @@ int tzr_solve_batch(tzr_ctx* ctx, const tzr_params* params, int B, const int32_t
 
 /* Device-resident batch of equally sized problems: src_dev/dst_dev hold B*n*3 doubles each
  * (problem-major), solutions_dev B tzr_solution, cliques_dev B*n int32 (may be NULL).  Asynchronous on
- * the context's stream; this is what bench.py's kernel-only timing and the multi-GPU shards drive. */
+ * the context's stream; this is what bench.py's kernel-only timing and the multi-GPU shards drive.  Exception: for
+ * n > 32768 the call synchronises the context's stream once, after the (L-1)-core peel, because the host needs the
+ * largest core of the batch to size the clique search. */
 int tzr_solve_batch_dev(tzr_ctx* ctx, const tzr_params* params, int B, int n, const double* src_dev,
                         const double* dst_dev, tzr_solution* solutions_dev, int32_t* cliques_dev);
 
@@ -269,7 +279,8 @@ int tzr_solve_batch_multi(const int32_t* devices, int n_devices, const tzr_param
  * the default CUDA-core kernel on B200: DESIGN.md 3.1), bit 9 (512) overrides it, bit 11 (2048) = the one-MUFU
  * CUDA-core variant (graph_strip3_kernel; bit-identical, FMA-pipe bound, 8 % slower), bit 13 (8192) = exact clique
  * search without the singleton-class path of the colouring (A/B), bit 12 (4096) = without the block colour bound (only
- * present in builds with -DTZR_BLOCK_BOUND). */
+ * present in builds with -DTZR_BLOCK_BOUND).  For n > 65535 bits 10 and 11 are ignored (both kernels' re-check queues
+ * pack a column index in 16 bits): the default graph kernel runs and counter [7] reports 0. */
 int tzr_ctx_set_flags(tzr_ctx* ctx, uint32_t flags);
 int64_t tzr_ctx_filter_mismatches(tzr_ctx* ctx);
 /* Number of pairs of the most recent graph build that needed the exact FP64 re-check. */
@@ -278,7 +289,8 @@ int64_t tzr_ctx_filter_rechecks(tzr_ctx* ctx);
  * search nodes, [3] reduce rounds, [4] vertices scanned by reduce rounds, [5] colourings, [6] vertices coloured,
  * [7] problems whose graph was built by the tensor-core kernel, [8]-[10] clock cycles of the exact search in the root
  * colour bound / degree rules / colourings, [11] slowest root (ns << 16 | vertex), [12] summed root time (ns),
- * [13] roots above 1 ms, [14] roots closed by the block colour bound. */
+ * [13] roots above 1 ms, [14] roots closed by the block colour bound, [15] n > 32768, PMC_EXACT: the largest number of
+ * vertices handed to the clique search after compaction to the (L-1)-core (0 on the n <= 32768 path). */
 int tzr_ctx_debug_counters(tzr_ctx* ctx, int64_t* out16);
 
 #ifdef __cplusplus

@@ -237,7 +237,9 @@ class Context:
                     # colourings, slowest root (ns, vertex), summed root time, roots above 1 ms
                     root_colour_cycles=int(out[8]), reduce_cycles=int(out[9]), colour_cycles=int(out[10]),
                     slowest_root_ns=int(out[11]) >> 16, slowest_root_vertex=int(out[11]) & 0xffff,
-                    root_ns_total=int(out[12]), roots_over_1ms=int(out[13]), block_bound_prunes=int(out[14]))
+                    root_ns_total=int(out[12]), roots_over_1ms=int(out[13]), block_bound_prunes=int(out[14]),
+                    # n > 32768 (flag 4): largest compacted (L-1)-core handed to the exact clique search in the batch
+                    clique_stage_vertices=int(out[15]))
 
     def kernel_launches(self) -> int:
         return int(lib().tzr_ctx_kernel_launches(self._h))

@@ -31,6 +31,9 @@ struct tzr_ctx {
   // device buffers (grow-only)
   DevBuf src, dst, sf, df, pk, opnd, tclist, gc, adj, deg, nedges, hclq, hsize, clq, L, alive, best_bits, alive_cnt, root_ctr, lock, flg, kfinal, tstart, stack, cv,
       centry, ps, pd, wgt, res, skey, sidx, sorted, rmask, tmask, sol, dbg, misc, sc_x, sc_r, sc_key, sc_idx, m_in, m_scratch, m_out, cert;
+  // n > kMaxN: scratch of the clique front end, and the clique buffers of the compacted (L-1)-cores
+  DevBuf large, compact;
+  LargeScratch lscr{};
   // pinned host staging
   void* h_pin = nullptr;
   size_t h_pin_cap = 0;
@@ -132,10 +135,40 @@ int effective_mode(const tzr_params& p) {
   return mode;
 }
 
+// Exact clique phase of a (B, n <= kMaxN) batch: a persistent grid that fills the GPU; its warps own the search scratch
+// (any problem).  Sets exact_ctas, max_depth and exact_conc of bt; returns the number of search warps.
+size_t exact_geometry(const tzr_ctx* ctx, int B, int n, Batch* bt) {
+  int G = clique_exact_grid(n, ctx->num_sms);
+  {
+    const long long roots = ((long long)B * n + 7) / 8;  // never more warps than root vertices
+    if ((long long)G > roots) G = (int)std::max<long long>(1, roots);
+  }
+  const size_t warps = (size_t)G * 8;
+  const size_t level_bytes = (size_t)2 * pitch32(n) * sizeof(uint32_t);
+  size_t depth = ((size_t)4 << 30) / (warps * level_bytes);
+  if (depth > 512) depth = 512;
+  if (depth > (size_t)n) depth = (size_t)n;
+  if (depth < 16) depth = 16;
+  bt->exact_ctas = G;
+  bt->max_depth = (int)depth;
+  {
+    // problems under search at a time: their bitsets should stay in the L2 together (~48 MB of the 126 MB: the
+    // stacks, the other lane's graph kernel and the two L2 partitions take the rest)
+    const size_t bits = (size_t)n * pitch32(n) * sizeof(uint32_t);
+    const size_t conc = ((size_t)48 << 20) / std::max<size_t>(bits, 1);
+    bt->exact_conc = (int)std::min<size_t>(std::max<size_t>(conc, 1), (size_t)B);
+  }
+  return warps;
+}
+
 // Size the workspace for a (B, n) batch and fill the Batch descriptor (src/dst left to the caller).
 int setup_batch(tzr_ctx* ctx, int B, int n, bool own_points, Batch* out, bool complete_graph = false) {
   if (B <= 0 || n <= 0) return TZR_ERR_INVALID_ARG;
-  if (n > kMaxN) return TZR_ERR_TOO_LARGE;
+  if (n > kMaxNGraph) {
+    ctx->last_error = "n = " + std::to_string(n) + " correspondences: at most " + std::to_string(kMaxNGraph) +
+                      " per problem are supported";
+    return TZR_ERR_TOO_LARGE;
+  }
   // the workspace is about to be re-used (and possibly re-allocated): the retained graph of the previous call is gone
   ctx->have_last = false;
   ctx->last_has_graph = false;
@@ -174,30 +207,16 @@ int setup_batch(tzr_ctx* ctx, int B, int n, bool own_points, Batch* out, bool co
   ENS(flg, (size_t)B * sizeof(int32_t));
   ENS(kfinal, (size_t)B * sizeof(int32_t));
   ENS(tstart, (size_t)B * sizeof(unsigned long long));
-  // exact phase geometry: a persistent grid that fills the GPU; its warps own the search scratch (any problem)
-  int G = clique_exact_grid(n, ctx->num_sms);
-  {
-    const long long roots = ((long long)B * n + 7) / 8;  // never more warps than root vertices
-    if ((long long)G > roots) G = (int)std::max<long long>(1, roots);
+  if (n <= kMaxN) {
+    const size_t warps = exact_geometry(ctx, B, n, &bt);
+    const size_t depth = (size_t)bt.max_depth, level_bytes = (size_t)2 * W32 * sizeof(uint32_t);
+    ENS(stack, warps * depth * level_bytes);
+    ENS(cv, std::max(warps, (size_t)4 * B) * (size_t)n * sizeof(int32_t));
+    ENS(centry, warps * depth * sizeof(int32_t));
+  } else {  // the exact search runs on the compacted cores (setup_clique_batch)
+    ENS(large, large_scratch_bytes(B, n));
+    ctx->lscr = large_scratch_carve(ctx->large.p, B, n);
   }
-  const size_t warps = (size_t)G * 8;
-  const size_t level_bytes = (size_t)2 * W32 * sizeof(uint32_t);
-  size_t depth = ((size_t)4 << 30) / (warps * level_bytes);
-  if (depth > 512) depth = 512;
-  if (depth > (size_t)n) depth = (size_t)n;
-  if (depth < 16) depth = 16;
-  bt.exact_ctas = G;
-  bt.max_depth = (int)depth;
-  {
-    // problems under search at a time: their bitsets should stay in the L2 together (~48 MB of the 126 MB: the
-    // stacks, the other lane's graph kernel and the two L2 partitions take the rest)
-    const size_t bits = n * W32 * sizeof(uint32_t);
-    const size_t conc = ((size_t)48 << 20) / std::max<size_t>(bits, 1);
-    bt.exact_conc = (int)std::min<size_t>(std::max<size_t>(conc, 1), (size_t)B);
-  }
-  ENS(stack, warps * depth * level_bytes);
-  ENS(cv, std::max(warps, (size_t)4 * B) * (size_t)n * sizeof(int32_t));
-  ENS(centry, warps * depth * sizeof(int32_t));
   bt.sort_cap = next_pow2_host(2 * n);
   ENS(ps, Bn * 3 * sizeof(double));
   ENS(pd, Bn * 3 * sizeof(double));
@@ -258,6 +277,7 @@ int setup_batch(tzr_ctx* ctx, int B, int n, bool own_points, Batch* out, bool co
   bt.mismatches = (unsigned long long*)ctx->dbg.p;
   bt.rechecks = (ctx->flags & 4u) ? (unsigned long long*)ctx->dbg.p + 1 : nullptr;
   bt.flags_dbg = ctx->flags;
+  if (n > kMaxNTc) bt.flags_dbg &= ~(1024u | 2048u);  // both re-check queues pack j in 16 bits: default graph kernel
   {
     static const double kappa_env = [] {
       const char* e = std::getenv("TZR_TC_KAPPA");
@@ -272,6 +292,66 @@ int setup_batch(tzr_ctx* ctx, int B, int n, bool own_points, Batch* out, bool co
   }
   bt.budget_ns = 0ull;
   *out = bt;
+  return TZR_OK;
+}
+
+// Clique buffers of a compacted batch: the B (L-1)-cores of a batch with n > kMaxN, nc <= kMaxN vertices each.  They
+// have their own region, so the full batch's bitset and clique stay in place for tzr_last_graph and the rotation stage.
+int setup_clique_batch(tzr_ctx* ctx, const Batch& full, int nc, Batch* out) {
+  const int B = full.B;
+  Batch cb{};
+  cb.B = B;
+  cb.n = nc;
+  const size_t Bn = (size_t)B * nc, W32 = (size_t)pitch32(nc);
+  const size_t warps = exact_geometry(ctx, B, nc, &cb);
+  const size_t depth = (size_t)cb.max_depth;
+  auto al = [](size_t x) { return (x + 255) & ~(size_t)255; };
+  const size_t sizes[] = {Bn * pitch64(nc) * sizeof(uint64_t),     // adj
+                          Bn * sizeof(int32_t),                    // deg
+                          (size_t)B * sizeof(unsigned long long),  // n_edges2
+                          Bn * kHeurRoots * sizeof(int32_t),       // hclq
+                          Bn * sizeof(int32_t),                    // clq
+                          (size_t)B * W32 * sizeof(uint32_t),      // alive
+                          (size_t)B * W32 * sizeof(uint32_t),      // best_bits
+                          (size_t)B * (kHeurRoots + 5) * sizeof(int32_t),  // hsize (kHeurRoots) | L | alive_cnt | root_ctr | lock | flags
+                          (size_t)B * sizeof(unsigned long long),  // t_start
+                          warps * depth * 2 * W32 * sizeof(uint32_t),                      // stack
+                          std::max(warps, (size_t)4 * B) * (size_t)nc * sizeof(int32_t),   // cv
+                          warps * depth * sizeof(int32_t)};                                // centry
+  size_t total = 0;
+  for (size_t x : sizes) total += al(x);
+  const int rc = ensure(ctx, ctx->compact, total);
+  if (rc != TZR_OK) return rc;
+  char* p = (char*)ctx->compact.p;
+  char* part[12];
+  for (int i = 0; i < 12; ++i) {
+    part[i] = p;
+    p += al(sizes[i]);
+  }
+  cb.adj = (uint64_t*)part[0];
+  cb.deg = (int32_t*)part[1];
+  cb.n_edges2 = (unsigned long long*)part[2];
+  cb.hclq = (int32_t*)part[3];
+  cb.clq = (int32_t*)part[4];
+  cb.alive = (uint32_t*)part[5];
+  cb.best_bits = (uint32_t*)part[6];
+  int32_t* small = (int32_t*)part[7];
+  cb.hsize = small;
+  cb.L = small + (size_t)B * kHeurRoots;
+  cb.alive_cnt = cb.L + B;
+  cb.root_ctr = cb.alive_cnt + B;
+  cb.lock = cb.root_ctr + B;
+  cb.flags = cb.lock + B;
+  cb.t_start = (unsigned long long*)part[8];
+  cb.stack = (uint32_t*)part[9];
+  cb.cv = (int32_t*)part[10];
+  cb.centry = (int32_t*)part[11];
+  cb.kcore_final = nullptr;
+  cb.mismatches = full.mismatches;
+  cb.rechecks = full.rechecks;
+  cb.flags_dbg = full.flags_dbg;
+  cb.budget_ns = full.budget_ns;
+  *out = cb;
   return TZR_OK;
 }
 
@@ -354,6 +434,53 @@ int l2_chunk(const tzr_ctx* ctx, int B, int n, const tzr_params& p) {
   return (int)c;
 }
 
+// Clique stage of a batch with n > kMaxN (clique_large.cu): greedy heuristic and core peel on the full graph, then
+// (PMC_EXACT) the existing search on the compacted (L-1)-cores.  The host waits once, after the peel, for the largest
+// core of the batch, which sizes the compacted batch.
+int run_clique_large(tzr_ctx* ctx, const Batch& bt, const tzr_params& p, int mode, cudaStream_t st, int* nl) {
+  const int B = bt.B;
+  const LargeScratch& ls = ctx->lscr;
+  const int k = launch_clique_large_front(bt, ls, mode, p.kcore_heuristic_threshold, st, ctx->num_sms);
+  if (k < 0) {
+    const int rc = check_launch(ctx, "clique front end (n > 32768)");
+    if (rc == TZR_OK) ctx->last_error = "clique front end (n > 32768): launch failed";
+    return TZR_ERR_CUDA;
+  }
+  *nl += k;
+  std::vector<int32_t> h(2 * (size_t)B);
+  CK(cudaMemcpyAsync(h.data(), ls.nsurv, (size_t)B * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+  CK(cudaMemcpyAsync(h.data() + B, bt.L, (size_t)B * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  int nc = 0;
+  for (int b = 0; b < B; ++b) {
+    const int core = h[b], L = h[B + b];
+    if (mode == 0 && core > kMaxN) {
+      ctx->last_error = "problem " + std::to_string(b) + ": the (L-1)-core of its inlier graph (L = " + std::to_string(L) +
+                        ", the greedy clique) has " + std::to_string(core) + " vertices; the exact search takes at most " +
+                        std::to_string(kMaxN) + " when n > " + std::to_string(kMaxN) +
+                        " (PMC_HEU and KCORE_HEU work at this size)";
+      return TZR_ERR_TOO_LARGE;
+    }
+    if (mode != 0 && L > kMaxN) {
+      ctx->last_error = "problem " + std::to_string(b) + ": the selected inlier set has " + std::to_string(L) +
+                        " vertices; the rotation stage takes at most " + std::to_string(kMaxN);
+      return TZR_ERR_TOO_LARGE;
+    }
+    nc = std::max(nc, core);
+  }
+  if (mode != 0 || nc == 0) return TZR_OK;  // no problem has an edge: the greedy result (L <= 1) stands
+  Batch cb;
+  int rc = setup_clique_batch(ctx, bt, nc, &cb);
+  if (rc) return rc;
+  CK(cudaMemsetAsync(cb.n_edges2, 0, (size_t)B * sizeof(unsigned long long), st));
+  launch_clique_compact(bt, ls, cb, st);
+  launch_degree(cb, st, true);
+  launch_clique(cb, p, 0, st, nl);
+  launch_clique_map_back(bt, ls, cb, st);
+  *nl += 3;
+  return check_launch(ctx, "compacted clique search");
+}
+
 // The fused device pipeline for one uniform batch.  src/dst must already be set in bt.
 // st: stream of the clique / rotation stages; sg: stream of prep + graph (== st for the single-lane form, otherwise
 // gdone is recorded on sg after the graph kernel and st waits for it).
@@ -364,6 +491,13 @@ int run_pipeline(tzr_ctx* ctx, Batch& bt, const tzr_params& p, cudaEvent_t* ev, 
       p.rotation_tim_graph > 1)
     return TZR_ERR_INVALID_ARG;
   const int mode = effective_mode(p);
+  if (bt.n > kMaxN && (p.estimate_scaling || mode == 3)) {
+    ctx->last_error = p.estimate_scaling
+                          ? "estimate_scaling is supported up to n = " + std::to_string(kMaxN) + " correspondences"
+                          : "inlier selection NONE hands all n > " + std::to_string(kMaxN) +
+                                " correspondences to the rotation stage, which takes at most " + std::to_string(kMaxN);
+    return TZR_ERR_TOO_LARGE;
+  }
   bt.beta = 2.0 * p.noise_bound * std::sqrt(p.cbar2);  // registration.cc:438
   // Params::max_clique_time_limit (seconds) -> device-side budget of the exact search
   bt.budget_ns = 0ull;
@@ -441,7 +575,12 @@ int run_pipeline(tzr_ctx* ctx, Batch& bt, const tzr_params& p, cudaEvent_t* ev, 
       nl += 2;
     }
     cudaEventRecord(ev[2], st);
-    launch_clique(bt, p, mode, st, &nl);
+    if (bt.n > kMaxN) {
+      const int rc = run_clique_large(ctx, bt, p, mode, st, &nl);
+      if (rc) return rc;
+    } else {
+      launch_clique(bt, p, mode, st, &nl);
+    }
   } else {
     if (sg != st) {
       cudaEventRecord(gdone, sg);
@@ -596,7 +735,8 @@ int tzr_ctx_destroy(tzr_ctx* ctx) {
                     &ctx->hclq, &ctx->hsize, &ctx->clq, &ctx->L, &ctx->alive, &ctx->best_bits, &ctx->alive_cnt, &ctx->root_ctr,
                     &ctx->lock, &ctx->flg, &ctx->kfinal, &ctx->tstart, &ctx->stack, &ctx->cv, &ctx->centry, &ctx->ps, &ctx->pd, &ctx->wgt,
                     &ctx->res, &ctx->skey, &ctx->sidx, &ctx->sorted, &ctx->rmask, &ctx->tmask, &ctx->sol, &ctx->dbg,
-                    &ctx->misc, &ctx->sc_x, &ctx->sc_r, &ctx->sc_key, &ctx->sc_idx, &ctx->m_in, &ctx->m_scratch, &ctx->m_out, &ctx->cert};
+                    &ctx->misc, &ctx->sc_x, &ctx->sc_r, &ctx->sc_key, &ctx->sc_idx, &ctx->m_in, &ctx->m_scratch, &ctx->m_out, &ctx->cert,
+                    &ctx->large, &ctx->compact};
   for (DevBuf* b : bufs)
     if (b->p) cudaFree(b->p);
   if (ctx->h_pin) cudaFreeHost(ctx->h_pin);
@@ -719,7 +859,12 @@ int tzr_max_clique(tzr_ctx* ctx, const uint64_t* adj_bits, int n, int mode, doub
   p.kcore_heuristic_threshold = kcore_thr;
   if (mode == 0 && time_limit_s > 0 && time_limit_s < 1e7) bt.budget_ns = (unsigned long long)(time_limit_s * 1e9);
   int nl = 1;
-  launch_clique(bt, p, mode, st, &nl);
+  if (n > kMaxN) {
+    rc = run_clique_large(ctx, bt, p, mode, st, &nl);
+    if (rc) return rc;
+  } else {
+    launch_clique(bt, p, mode, st, &nl);
+  }
   ctx->launches += nl;
   rc = check_launch(ctx, "max clique");
   if (rc) return rc;
@@ -869,7 +1014,8 @@ int tzr_solve_batch_dev(tzr_ctx* ctx, const tzr_params* params, int B, int n, co
     return e ? std::max(1, atoi(e)) : 1;
   }();
   std::vector<int> bounds{0};
-  const int nch = (B >= 64 * dev_chunks && !params->estimate_scaling) ? dev_chunks : 1;
+  // n > kMaxN: one chunk (the clique stage waits for the batch's largest core; its scratch covers the whole batch)
+  const int nch = (B >= 64 * dev_chunks && !params->estimate_scaling && n <= kMaxN) ? dev_chunks : 1;
   for (int c = 1; c <= nch; ++c) bounds.push_back((int)((long long)B * c / nch));
   rc = run_chunked(ctx, bt, *params, bounds, nullptr);
   if (rc) return rc;
@@ -919,7 +1065,7 @@ static int solve_uniform_host(tzr_ctx* ctx, const tzr_params* params, int B, int
   // PCIe moves a problem ~3x faster than the kernels consume it, so only the first chunk's copy is exposed: it is
   // kept small (B/32) and the later chunks grow (3B/32, B/8, then B/4 each) to keep launch tails few.
   std::vector<int> bounds{0};
-  if (B >= 64 && !params->estimate_scaling) {
+  if (B >= 64 && !params->estimate_scaling && n <= kMaxN) {
     const int unit = std::max(8, B / 32);
     const int sizes[3] = {unit, 3 * unit, 4 * unit};
     for (int k = 0; bounds.back() < B; ++k) {

@@ -29,6 +29,9 @@ constexpr int kMatchMaxDim = 128;   // feature dimension limit of the matcher's 
 constexpr double kTcKappa = 12.0;   // bound on the tensor-core Gram error |a' - a| in units of 2^-24 * D^2 (D = largest distance
                                     // inside the cloud); measured with csrc/tc_probe (profiles/), x4 safety
 constexpr int kMaxN = 32768;        // per-problem size limit of the shared-memory clique kernels
+constexpr int kMaxNGraph = 131072;  // per-problem size limit of every entry point: above kMaxN the clique stage runs on
+                                    // the compacted (L-1)-core (clique_large.cu); one problem's bitset is then 2 GiB
+constexpr int kMaxNTc = 65535;      // the re-check queues of the tensor-core and v7 graph kernels pack i << 16 | j
 
 // Per-problem constants of the FP32 filter (see graph_build.cu).
 struct GraphConsts {
@@ -145,6 +148,20 @@ static __device__ __noinline__ bool edge_exact_scale(const double* __restrict__ 
   return fabs(__dsub_rn(ratio, s_hat)) <= alpha;
 }
 
+// Scratch of the clique front end of problems with n > kMaxN (clique_large.cu).  Per-problem arrays are indexed by
+// the full n; bt.alive holds the survivors of the last peel.
+struct LargeScratch {
+  int32_t* hl;       // B*kHeurRoots*2n: member list | in-P degrees of each greedy heuristic
+  int32_t* dcur;     // B*n: degree inside the surviving set while peeling
+  uint32_t* dying;   // B*pitch32(n): vertices removed in the current peel round
+  int32_t* k;        // B: peel threshold (a vertex with fewer than k surviving neighbours is removed); < 0: problem skipped
+  int32_t* lo;       // B: core-number bisection (KCORE_HEU): the lo-core is non-empty ...
+  int32_t* hi;       // B: ... and the hi-core is empty
+  int32_t* surv;     // B*n: survivors of the last peel in ascending order
+  int32_t* nsurv;    // B: survivors of the last peel
+  unsigned int* total;  // 3: vertices removed so far in the running peel (its convergence test) | grid barrier (2)
+};
+
 // kernels (defined in the .cu files) -------------------------------------------------------------
 void launch_prep(const Batch& bt, cudaStream_t st);
 int launch_graph(const Batch& bt, cudaStream_t st, int num_sms);  // returns the number of kernels launched
@@ -165,6 +182,20 @@ size_t clique_heur_smem(int n);
 size_t clique_peel_smem(int n);
 size_t clique_exact_smem(int n);
 int clique_exact_grid(int n, int num_sms);  // CTAs of the persistent exact-phase grid on the current device
+// clique_large.cu: front end of the clique stage for kMaxN < n <= kMaxNGraph
+size_t large_scratch_bytes(int B, int n);
+LargeScratch large_scratch_carve(void* base, int B, int n);
+// Greedy heuristic on the full graph, then per mode: PMC_EXACT peels to the (L-1)-core and lists the survivors
+// (ls.surv / ls.nsurv); PMC_HEU leaves the best greedy clique in L / clq; KCORE_HEU finds the max core by bisection and
+// leaves the innermost core in L / clq when it exceeds the threshold (kcore_final), the greedy clique otherwise.
+// Returns the number of kernels launched, -1 if a launch failed.
+int launch_clique_large_front(const Batch& bt, const LargeScratch& ls, int mode, double kcore_thr, cudaStream_t st,
+                              int num_sms);
+// PMC_EXACT, after launch_clique_large_front: cb.adj = the sub-graph induced by the survivors (cb.n = the largest
+// survivor count of the batch, shorter problems padded with isolated vertices) ...
+void launch_clique_compact(const Batch& bt, const LargeScratch& ls, const Batch& cb, cudaStream_t st);
+// ... and, after launch_clique on cb, its clique in the indices of the full problem (L, clq, flags of bt).
+void launch_clique_map_back(const Batch& bt, const LargeScratch& ls, const Batch& cb, cudaStream_t st);
 
 // stand-alone stage helpers used by the per-stage C-ABI entry points
 void launch_gnc_only(int alg, const double* src, const double* dst, int m, double noise_bound, double gnc_factor,
